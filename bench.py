@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the pseudo-label generator hot path (BASELINE.json metric: scenes/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one pass of the whole hot path over one batch of synthetic ScanNet-shaped scenes
@@ -348,6 +348,24 @@ def ncu_traffic(kernel_regex, args):
     return None, "no ncu capture of this workload committed"
 
 
+OUTPUT_FIELDS = ("sem", "inst", "prob", "mu", "var")
+
+
+def dump_outputs(outs, out_dir, max_bytes=64 << 20):
+    """Write what one step of the timed path returned, so that two builds can be compared output for output: for
+    each field of the per-scene (sem, inst, prob, mu, var) tuples, the scenes' arrays concatenated in job order as
+    float32 <out_dir>/<field>.npy (the integer labels are small, so float32 holds them exactly).  A field longer than
+    its share of max_bytes is cut to a uniform sample of positions drawn with a fixed seed, kept in position order:
+    the same positions on every run with the same arguments, and the same for sem / inst / prob."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (max_bytes // len(OUTPUT_FIELDS) - 128) // 4       # float32 elements per file (128: the .npy header)
+    for i, name in enumerate(OUTPUT_FIELDS):
+        a = torch.cat([o[i].reshape(-1) for o in outs]).float().cpu().numpy()
+        if len(a) > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu(args):
     rank, world, local = dist_env()
     import torch.distributed as dist
@@ -445,6 +463,8 @@ def run_gpu(args):
     clocks = sampler.stop()
     ms_step = ms_total / args.steps
     value = len(ids) / (ms_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(outs, args.dump_outputs)
 
     # ---- end to end: pinned host inputs -> device -> hot path -> host ----------------------------
     pinned, h2d = [], 0
@@ -633,7 +653,14 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=None, help="seconds of CPU work per step of the CPU arm")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs to DIR/<sem|inst|prob|mu|var>.npy (float32, "
+                         "64 MB at most: longer fields are a fixed seeded sample); single-process GPU arm only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or dist_env()[1] > 1):
+        ap.error("--dump-outputs needs the GPU arm in a single process")
     # stdout carries exactly ONE line (the JSON); whatever libraries print there (NCCL prints its version banner
     # to stdout at communicator creation) goes to stderr instead
     global _RESULT_OUT

@@ -11,13 +11,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from gapro_b200.engine import SceneInputs, get_engine  # noqa: E402
 from tests.conftest import rel_err  # noqa: E402
-from tests.golden.make_golden_fullsize import SCENES, scene_args  # noqa: E402
+from tests.golden.make_golden_fullsize import SCENES, load_scene, scene_args  # noqa: E402
 
 dev = torch.device("cuda:0")
 TAG = sys.argv[1] if len(sys.argv) > 1 else "c4"
-gold = np.load(os.path.join(ROOT, "tests", "golden", f"scene_{TAG}_full.npz"))
 cfg_name, seed, nseed = SCENES[TAG]
 args = scene_args(cfg_name, seed)
+gold = load_scene(TAG, args[2])
 T = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a)).to(dt).to(dev)
 sc = SceneInputs(T(args[0], torch.float64), T(args[1], torch.float32), T(args[2], torch.int64), T(args[3], torch.int64),
                  T(args[4], torch.float32), T(args[5], torch.float32), T(args[6], torch.float32), T(args[7], torch.float32),

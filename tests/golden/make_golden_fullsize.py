@@ -11,6 +11,8 @@ committed rather than recomputed by the GPU tests):
 
   scene_c5_full.npz    one configs[4] scene (1M points, 125 boxes, 349 GP regions up to M = 3587; ~3 CPU-hours)
 
+The scene files hold the point labels once per superpoint (sem_spp / inst_spp / prob_spp); load_scene expands them.
+
     python tests/golden/make_golden_fullsize.py [gp8k] [c1] [c3] [c4] [c5]
 
 Like make_golden.py these pin the CUDA path to the ORACLE at full size; the oracle's scene pipeline is
@@ -59,15 +61,38 @@ def make_gp8k():
           f"({time.time() - t0:.0f}s)")
 
 
+def to_superpoints(spp, point_labels):
+    """sem / inst / prob of a scene are broadcast from its superpoints: one value per superpoint, in the order of
+    mu / var (np.unique of the raw superpoint ids).  Keeps the full-size fixtures small."""
+    dense = np.unique(spp, return_inverse=True)[1]
+    out = []
+    for a in point_labels:
+        s = np.zeros(dense.max() + 1, a.dtype)
+        s[dense] = a
+        assert (s[dense] == a).all(), "a label differs inside a superpoint"
+        out.append(s)
+    return out
+
+
+def load_scene(tag, spp):
+    """scene_<tag>_full.npz with sem / inst / prob expanded from superpoints back to the scene's points."""
+    gold = dict(np.load(os.path.join(HERE, f"scene_{tag}_full.npz")))
+    dense = np.unique(spp, return_inverse=True)[1]
+    for k in ("sem", "inst", "prob"):
+        gold[k] = gold.pop(k + "_spp")[dense]
+    return gold
+
+
 def make_scene(tag):
     cfg_name, seed, nseed = SCENES[tag]
     args = scene_args(cfg_name, seed)
     t0 = time.time()
     res, dbg = O.gen_pseudo_label_oracle(*args, thresh_spp_occu=0.999, noise_seed=nseed, return_debug=True)
     margins = [np.abs(r["res"]["prob64"] - 0.5).min() for r in dbg["regions"]]
+    sem, inst, prob = to_superpoints(args[2], (res[0].astype(np.int8), res[1].astype(np.int16), res[2]))
     # competition margin: |new confidence - confidence being replaced| over all merges, from a replay
-    np.savez_compressed(os.path.join(HERE, f"scene_{tag}_full.npz"), sem=res[0].astype(np.int8), inst=res[1].astype(np.int16),
-                        prob=res[2], mu=res[3], var=res[4], digest=np.array(input_digest(args)),
+    np.savez_compressed(os.path.join(HERE, f"scene_{tag}_full.npz"), sem_spp=sem, inst_spp=inst,
+                        prob_spp=prob, mu=res[3], var=res[4], digest=np.array(input_digest(args)),
                         n_regions=np.array(len(dbg["regions"])), min_margin=np.array(min(margins) if margins else 1.0),
                         max_m=np.array(max((len(r["b1_inds"]) + len(r["b2_inds"]) for r in dbg["regions"]), default=0)),
                         occ_spp=np.packbits(dbg["occ_spp"], axis=1))

@@ -530,10 +530,10 @@ def test_gp_region_of_8k_superpoints_matches_golden(dev, lib, tcgen05, monkeypat
 def test_full_size_scene_matches_offline_oracle_fixture(engine, dev, tag):
     """One whole configs[1] scene (150k points, 93 GP regions) and scene 0 of the configs[2] bench batch (212k
     points, regions up to M = 1126): labels bit-exact, mu / var 1e-4 (asserted 1e-5) against the fp64 oracle."""
-    from tests.golden.make_golden_fullsize import SCENES, input_digest, scene_args
-    gold = np.load(os.path.join(GOLD_DIR, f"scene_{tag}_full.npz"))
+    from tests.golden.make_golden_fullsize import SCENES, input_digest, load_scene, scene_args
     cfg_name, seed, nseed = SCENES[tag]
     args = scene_args(cfg_name, seed)
+    gold = load_scene(tag, args[2])
     assert input_digest(args) == str(gold["digest"])        # same synthetic inputs as the fixture was made from
     from gapro_b200.engine import SceneInputs
     T = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a)).to(dt).to(dev)
@@ -751,13 +751,13 @@ def test_small_region_kernel_against_numpy_mirror_and_batched_path(dev, lib, mon
 
 def _full_scene_against_fixture(engine, dev, tag, min_max_m, tol=1e-5, prob_tol=2e-6):
     from gapro_b200.engine import SceneInputs
-    from tests.golden.make_golden_fullsize import SCENES, input_digest, scene_args
+    from tests.golden.make_golden_fullsize import SCENES, input_digest, load_scene, scene_args
     path = os.path.join(GOLD_DIR, f"scene_{tag}_full.npz")
     if not os.path.exists(path):
         pytest.skip(f"{path} not generated (tests/golden/make_golden_fullsize.py {tag})")
-    gold = np.load(path)
     cfg_name, seed, nseed = SCENES[tag]
     args = scene_args(cfg_name, seed)
+    gold = load_scene(tag, args[2])
     assert input_digest(args) == str(gold["digest"])
     T = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a)).to(dt).to(dev)
     sc = SceneInputs(T(args[0], torch.float64), T(args[1], torch.float32), T(args[2], torch.int64), T(args[3], torch.int64),

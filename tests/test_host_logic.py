@@ -232,6 +232,34 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert d["value"] > 0 and "workload" in d["config"]
 
 
+def test_bench_dump_outputs_is_float32_seeded_and_capped(tmp_path):
+    """bench.py --dump-outputs: one float32 file per output field with the scenes in job order; a field over its share
+    of the byte cap is cut to the same positions on every call, shared by the per-point fields."""
+    import bench
+    g = torch.Generator().manual_seed(0)
+    outs, off = [], 0
+    for n, s in ((3000, 40), (5000, 70)):
+        # prob carries the point's position in the job, so the sampled positions can be read back from it
+        outs.append((torch.randint(-100, 19, (n,), dtype=torch.int32, generator=g),
+                     torch.randint(-100, 30, (n,), dtype=torch.int32, generator=g),
+                     torch.arange(off, off + n, dtype=torch.float32), torch.rand(s, generator=g), torch.rand(s, generator=g)))
+        off += n
+    cap = 5 * (128 + 4 * 1000)                  # 1000 float32 values per file
+    for d in ("a", "b"):
+        bench.dump_outputs(outs, str(tmp_path / d), max_bytes=cap)
+    got = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in bench.OUTPUT_FIELDS}
+    for k, a in got.items():
+        assert a.dtype == np.float32 and np.array_equal(a, np.load(tmp_path / "b" / f"{k}.npy")), k
+    assert sum(os.path.getsize(tmp_path / "a" / f"{k}.npy") for k in got) <= cap
+    full = {k: torch.cat([o[i] for o in outs]).numpy() for i, k in enumerate(bench.OUTPUT_FIELDS)}
+    for k in ("mu", "var"):
+        assert np.array_equal(got[k], full[k])
+    pos = got["prob"].astype(np.int64)
+    assert len(pos) == 1000 and (np.diff(pos) > 0).all()
+    for k in ("sem", "inst"):
+        assert np.array_equal(got[k], full[k][pos].astype(np.float32)), k
+
+
 def test_bench_gpu_arm_refuses_to_run_without_a_gpu():
     import subprocess
     import sys
