@@ -1370,11 +1370,6 @@ k_region_init(const Region* __restrict__ regs, int D, const float* __restrict__ 
 inline int ceil64(int x) { return (x + 63) / 64 * 64; }
 
 // ---- tcgen05 path configuration (development knobs; defaults are what the parity suite runs with) -----------
-static int oz_digits() {
-    int s = 8;      // 2^-55 truncation per operand (ozaki.cu); 6 -> 2^-41, 7 -> 2^-48
-    if (const char* e = getenv("GAPRO_GP_OZAKI_S")) s = atoi(e);
-    return s < 5 ? 5 : (s > 8 ? 8 : s);
-}
 static int oz_min_rows() {
     // GAPRO_GP_OZAKI=1: regions with at least this many padded training rows run their tile products on tcgen05
     // (8 digits).  Opt-in: the digit-plane products are accurate relative to row-max x column-max x K, float64 is
@@ -1421,7 +1416,7 @@ size_t region_core_doubles(const Region& r, int D) {
 }
 size_t region_doubles(const Region& r, int D) {
     size_t d = region_core_doubles(r, D);
-    if (r.oz) d += (size_t)gapro_align_up((size_t)oz_region_doubles(r.Mp, oz_digits()), 32);
+    if (r.oz) d += (size_t)gapro_align_up((size_t)oz_region_doubles(r.Mp), 32);
     return d;
 }
 
@@ -1638,26 +1633,18 @@ struct Driver {
         return p;
     }
 
-    int ozS = 6;      // digits per operand of the tcgen05 path
-
     void oz_slice(int mat, int flags, int buf, const GpParams& p) {
-        k_oz_zero_b<<<tb.n_oz_vb, 64, 0, stream>>>(tb.regs, tb.oz_vb, ws, ozS, buf);
-        k_oz_vecmax_b<<<dim3(tb.n_oz_vb, (tb.oz_max_m + OZ_KCH - 1) / OZ_KCH), 256, 0, stream>>>(tb.regs, tb.oz_vb, p, ws, ozS,
+        k_oz_zero_b<<<tb.n_oz_vb, 64, 0, stream>>>(tb.regs, tb.oz_vb, ws, buf);
+        k_oz_vecmax_b<<<dim3(tb.n_oz_vb, (tb.oz_max_m + OZ_KCH - 1) / OZ_KCH), 256, 0, stream>>>(tb.regs, tb.oz_vb, p, ws,
                                                                                                 mat, flags, buf);
-        if (ozS == 5) k_oz_slice_b<5><<<tb.n_oz_blk, 256, 0, stream>>>(tb.regs, tb.oz_blk, p, ws, mat, flags, buf);
-        else if (ozS == 6) k_oz_slice_b<6><<<tb.n_oz_blk, 256, 0, stream>>>(tb.regs, tb.oz_blk, p, ws, mat, flags, buf);
-        else if (ozS == 7) k_oz_slice_b<7><<<tb.n_oz_blk, 256, 0, stream>>>(tb.regs, tb.oz_blk, p, ws, mat, flags, buf);
-        else k_oz_slice_b<8><<<tb.n_oz_blk, 256, 0, stream>>>(tb.regs, tb.oz_blk, p, ws, mat, flags, buf);
+        k_oz_slice_b<<<tb.n_oz_blk, 256, 0, stream>>>(tb.regs, tb.oz_blk, p, ws, mat, flags, buf);
         g_launches += 3;
     }
     template <int PH>
     void oz_gemm(bool lower, int abuf, int bbuf, const GpParams& p) {
         const int4* tiles = lower ? tb.oz_lower : tb.oz_full;
         const int n = lower ? tb.n_oz_lower : tb.n_oz_full;
-        if (ozS == 5) k_oz_gemm_b<5, PH><<<n, oz::OZ_THREADS, oz::oz_smem_bytes(5), stream>>>(tb.regs, tiles, p, ws, abuf, bbuf);
-        else if (ozS == 6) k_oz_gemm_b<6, PH><<<n, oz::OZ_THREADS, oz::oz_smem_bytes(6), stream>>>(tb.regs, tiles, p, ws, abuf, bbuf);
-        else if (ozS == 7) k_oz_gemm_b<7, PH><<<n, oz::OZ_THREADS, oz::oz_smem_bytes(7), stream>>>(tb.regs, tiles, p, ws, abuf, bbuf);
-        else k_oz_gemm_b<8, PH><<<n, oz::OZ_THREADS, oz::oz_smem_bytes(8), stream>>>(tb.regs, tiles, p, ws, abuf, bbuf);
+        k_oz_gemm_b<PH><<<n, oz::OZ_THREADS, oz::oz_smem_bytes(OZ_S), stream>>>(tb.regs, tiles, p, ws, abuf, bbuf);
         ++g_launches;
     }
     // phase PH of the large regions: slice the operands it contracts, then the tcgen05 tile product
@@ -2090,26 +2077,17 @@ static int set_kernel_attributes() {
     if (rc == GAPRO_OK) rc = allow_smem(k_gemm<PH_GL>, GEMM_SMEM);
     if (rc == GAPRO_OK) rc = allow_smem(k_gemm<PH_Y>, GEMM_SMEM);
     if (rc == GAPRO_OK) rc = allow_smem(k_gemm<PH_GK>, GEMM_SMEM);
-#define OZ_ATTR(S_)                                                                                     \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_A>, oz::oz_smem_bytes(S_));                  \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_B>, oz::oz_smem_bytes(S_));                  \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_GA>, oz::oz_smem_bytes(S_));                 \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_GT>, oz::oz_smem_bytes(S_));                 \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_GC>, oz::oz_smem_bytes(S_));                 \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_GL>, oz::oz_smem_bytes(S_));                 \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_Y>, oz::oz_smem_bytes(S_));                  \
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<S_, PH_GK>, oz::oz_smem_bytes(S_));
-    OZ_ATTR(5)
-    OZ_ATTR(6)
-    OZ_ATTR(7)
-    OZ_ATTR(8)
-#undef OZ_ATTR
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_A>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_B>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_GA>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_GT>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_GC>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_GL>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_Y>, oz::oz_smem_bytes(OZ_S));
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_gemm_b<PH_GK>, oz::oz_smem_bytes(OZ_S));
     if (rc == GAPRO_OK) rc = allow_smem(k_oz_vecmax_b, 0);
     if (rc == GAPRO_OK) rc = allow_smem(k_oz_zero_b, 0);
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_slice_b<5>, 0);
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_slice_b<6>, 0);
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_slice_b<7>, 0);
-    if (rc == GAPRO_OK) rc = allow_smem(k_oz_slice_b<8>, 0);
+    if (rc == GAPRO_OK) rc = allow_smem(k_oz_slice_b, 0);
     if (rc == GAPRO_OK) rc = allow_smem(k_kgrad<6, 4>, kgrad_smem<6, 4>());
     if (rc == GAPRO_OK) rc = allow_smem(k_kgrad<8, 4>, kgrad_smem<8, 4>());
     if (rc == GAPRO_OK) rc = allow_smem(k_kgrad_wide<1>, kgrad_wide_smem<1>());
@@ -2177,7 +2155,6 @@ static int run_regions(const float* feats_spp, int32_t D, std::vector<Region>& a
                 d.stream = d.s_hi;
                 if (g > 0 && !getenv("GAPRO_GP_NO_STAGGER")) d.ev_prev_swept = g_pool.swept[g - 1];
             }
-            d.ozS = oz_digits();
             d.careful = careful;
             if (careful) d.tb_orig = groups[g][0].orig;
             d.D = D;

@@ -13,17 +13,21 @@
 enum OzMat { OM_LINV = 0, OM_KZX, OM_T, OM_A, OM_BM, OM_GA };
 enum OzBuf { OB_LR = 0, OB_LC, OB_X1, OB_X2, OB_X3, OB_COUNT };
 
+// Digits per operand: 8, a 2^-55 truncation per operand (ozaki.cu).  6 and 7 digits (2^-41, 2^-48) miss the 1e-6
+// parity bar on the golden regions (DESIGN.md section 4.1).
+constexpr int OZ_S = 8;
+
 __host__ __device__ inline int oz_rb(int Mp) { return (Mp + 127) / 128 * 2; }                // 64-vector blocks per plane row
 __host__ __device__ inline size_t oz_plane_bytes(int Mp) { return (size_t)(Mp / 64) * oz_rb(Mp) * oz::OZ_BLK; }
-__host__ __device__ inline size_t oz_buf_bytes(int Mp, int S) { return (size_t)S * oz_plane_bytes(Mp); }
-__host__ __device__ inline long long oz_region_doubles(int Mp, int S) {
-    return (long long)OB_COUNT * ((long long)(oz_buf_bytes(Mp, S) / 8) + (long long)oz_rb(Mp) * 64);
+__host__ __device__ inline size_t oz_buf_bytes(int Mp) { return (size_t)OZ_S * oz_plane_bytes(Mp); }
+__host__ __device__ inline long long oz_region_doubles(int Mp) {
+    return (long long)OB_COUNT * ((long long)(oz_buf_bytes(Mp) / 8) + (long long)oz_rb(Mp) * 64);
 }
-__device__ __forceinline__ uint8_t* oz_buf(double* ws, const Region& R, int S, int b) {
-    return reinterpret_cast<uint8_t*>(ws + R.oz_base) + (size_t)b * oz_buf_bytes(R.Mp, S);
+__device__ __forceinline__ uint8_t* oz_buf(double* ws, const Region& R, int b) {
+    return reinterpret_cast<uint8_t*>(ws + R.oz_base) + (size_t)b * oz_buf_bytes(R.Mp);
 }
-__device__ __forceinline__ double* oz_scale(double* ws, const Region& R, int S, int b) {
-    return ws + R.oz_base + (long long)OB_COUNT * (long long)(oz_buf_bytes(R.Mp, S) / 8) + (long long)b * oz_rb(R.Mp) * 64;
+__device__ __forceinline__ double* oz_scale(double* ws, const Region& R, int b) {
+    return ws + R.oz_base + (long long)OB_COUNT * (long long)(oz_buf_bytes(R.Mp) / 8) + (long long)b * oz_rb(R.Mp) * 64;
 }
 __device__ __forceinline__ const double* oz_src(const Layout& lay, const double* base, const Region& R, int mat, int& ld) {
     switch (mat) {
@@ -55,15 +59,15 @@ constexpr int OZ_KCH = 512;      // k-range of one k_oz_vecmax_b CTA
 __device__ __forceinline__ double oz_pow2(double m) { return (m > 0.0 && m < 1e300) ? ldexp(1.0, ilogb(m) + 1) : 1.0; }
 
 __global__ void __launch_bounds__(64)
-k_oz_zero_b(const Region* __restrict__ regs, const int2* __restrict__ vblocks, double* __restrict__ ws, int S, int buf) {
+k_oz_zero_b(const Region* __restrict__ regs, const int2* __restrict__ vblocks, double* __restrict__ ws, int buf) {
     const int2 vb = vblocks[blockIdx.x];
     const Region R = regs[vb.x];
-    oz_scale(ws, R, S, buf)[vb.y * 64 + threadIdx.x] = 0.0;
+    oz_scale(ws, R, buf)[vb.y * 64 + threadIdx.x] = 0.0;
 }
 
 __global__ void __launch_bounds__(256)
 k_oz_vecmax_b(const Region* __restrict__ regs, const int2* __restrict__ vblocks, GpParams prm, double* __restrict__ ws,
-              int S, int mat, int flags, int buf) {
+              int mat, int flags, int buf) {
     __shared__ double red[4][64];
     const int2 vb = vblocks[blockIdx.x];
     const Region R = regs[vb.x];
@@ -75,7 +79,7 @@ k_oz_vecmax_b(const Region* __restrict__ regs, const int2* __restrict__ vblocks,
     int ld;
     const double* X = oz_src(lay, base, R, mat, ld);
     const double* ks = (flags & OZF_GV) ? base + lay.gv : nullptr;
-    unsigned long long* mx = reinterpret_cast<unsigned long long*>(oz_scale(ws, R, S, buf));
+    unsigned long long* mx = reinterpret_cast<unsigned long long*>(oz_scale(ws, R, buf));
     if (!(flags & OZF_TRANS)) {
         const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
         for (int r = 0; r < 8; ++r) {
@@ -101,62 +105,32 @@ k_oz_vecmax_b(const Region* __restrict__ regs, const int2* __restrict__ vblocks,
     }
 }
 
-// one 4 KB block (64 vectors x 64 k) of each of the S digit planes per CTA; table entry (region, kb, rb)
-template <int S>
+// one 4 KB block (64 vectors x 64 k) of each of the OZ_S digit planes per CTA; table entry (region, kb, rb)
 __global__ void __launch_bounds__(256)
 k_oz_slice_b(const Region* __restrict__ regs, const int4* __restrict__ blocks, GpParams prm, double* __restrict__ ws,
              int mat, int flags, int buf) {
-    constexpr int LD = 68;
-    __shared__ double blk[64 * LD + 8];
     const int4 e4 = blocks[blockIdx.x];
     const Region R = regs[e4.x];
-    const int kb = e4.y, rb = e4.z;
     const Layout lay = make_layout(R.Mp, R.Np, R.Wp, prm.D);
     const double* base = ws + R.base;
     int ld;
     const double* X = oz_src(lay, base, R, mat, ld);
     const double* ks = (flags & OZF_GV) ? base + lay.gv : nullptr;
-    const double* scale = oz_scale(ws, R, S, buf);
-    const int M = R.M, v0 = rb * 64, k0 = kb * 64;
-    const bool trans = flags & OZF_TRANS;
-    for (int e = threadIdx.x; e < 64 * 64; e += 256) {
-        const int a = e >> 6, b = e & 63;          // b runs along the contiguous direction of the source
-        const int v = trans ? b : a, k = trans ? a : b;
-        double x = 0.0;
-        if (oz_valid(v0 + v, k0 + k, M, flags)) {
-            x = trans ? X[(size_t)(k0 + k) * ld + v0 + v] : X[(size_t)(v0 + v) * ld + k0 + k];
-            if (ks) x *= ks[k0 + k];
-        }
-        blk[v * LD + k + (k >> 4)] = x;
-    }
-    __syncthreads();
-    const int t = threadIdx.x;
-    const int atom = t >> 5, r = (t & 31) >> 2, c = t & 3;
-    const int v = 8 * atom + r;
-    const double inv = (v0 + v < M) ? 64.0 / oz_pow2(scale[v0 + v]) : 0.0;      // exact: a power of two
-    double y[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) y[j] = blk[v * LD + 16 * c + j + c] * inv;      // |y| < 64
-    const size_t plane = oz_plane_bytes(R.Mp);
-    uint8_t* dst = oz_buf(ws, R, S, buf) + ((size_t)kb * oz_rb(R.Mp) + rb) * oz::OZ_BLK + atom * 512 + r * 64 +
-                   ((c ^ ((r >> 1) & 3)) * 16);
-    oz::emit_digits<S>(y, dst, plane);
+    const double* scale = oz_scale(ws, R, buf);
+    const int M = R.M;
+    oz::oz_slice_block<OZ_S>(
+        X, ld, flags & OZF_TRANS, ks, e4.y, e4.z, [&](int v, int k) { return oz_valid(v, k, M, flags); },
+        [&](int v) { return v < M ? 64.0 / oz_pow2(scale[v]) : 0.0; }, 1.0,      // exact: a power of two
+        oz_buf(ws, R, buf), R.Mp / 64, oz_rb(R.Mp));      // oz_plane_bytes(R.Mp) per plane
 }
 
 // C tile (128 x 64) of phase PH for one large region; table entry (region, ti, tj)
-template <int S, int PH>
+template <int PH>
 __global__ void __launch_bounds__(oz::OZ_THREADS, 1)
 k_oz_gemm_b(const Region* __restrict__ regs, const int4* __restrict__ tiles, GpParams prm, double* __restrict__ ws,
             int abuf, int bbuf) {
     using namespace oz;
     extern __shared__ __align__(1024) uint8_t oz_smem_b[];
-    constexpr int STAGE = oz_stage_bytes(S);
-    constexpr int NST = oz_stages(S);
-    uint8_t* smem = (uint8_t*)(((uintptr_t)oz_smem_b + 1023) & ~(uintptr_t)1023);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + NST * STAGE);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * NST + 1);
-    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + NST), tfull = smem_u32(bars + 2 * NST);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int4 t4 = tiles[blockIdx.x];
     const Region R = regs[t4.x];
     const int ti = t4.y, tj = t4.z;
@@ -166,190 +140,89 @@ k_oz_gemm_b(const Region* __restrict__ regs, const int4* __restrict__ tiles, GpP
     if (PH == PH_A || PH == PH_GA) k1 = min(kbt, 2 * ti + 2);             // A operand lower triangular: k <= i
     if (PH == PH_B || PH == PH_GC || PH == PH_GK) k0 = min(kbt, 2 * ti);  // A operand = transposed lower: k >= i
     if (PH == PH_Y) k0 = min(kbt, tj);                                    // B operand = L^-1 columns: k >= j
-    const int nkb = k1 - k0;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NST; ++s) {
-            mbar_init(full0 + 8 * s, 1);
-            mbar_init(empty0 + 8 * s, 1);
-        }
-        mbar_init(tfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-    const int rbP = oz_rb(R.Mp);
-    const size_t plane = oz_plane_bytes(R.Mp);
-
-    if (warp == 0) {
-        if (lane == 0) {
-            const uint8_t* ap = oz_buf(ws, R, S, abuf);
-            const uint8_t* bp = oz_buf(ws, R, S, bbuf);
-            for (int i = 0; i < nkb; ++i) {
-                const int st = i % NST;
-                mbar_wait(empty0 + 8 * st, ((i / NST) & 1) ^ 1);
-                mbar_expect_tx(full0 + 8 * st, (uint32_t)STAGE);
-                const uint32_t dst = smem_u32(smem + st * STAGE);
-                const uint8_t* ga = ap + ((size_t)(k0 + i) * rbP + 2 * ti) * OZ_BLK;
-                const uint8_t* gb = bp + ((size_t)(k0 + i) * rbP + tj) * OZ_BLK;
-#pragma unroll
-                for (int s = 0; s < S; ++s) {
-                    bulk_g2s(dst + s * 2 * OZ_BLK, ga + s * plane, 2 * OZ_BLK, full0 + 8 * st);
-                    bulk_g2s(dst + S * 2 * OZ_BLK + s * OZ_BLK, gb + s * plane, OZ_BLK, full0 + 8 * st);
-                }
-            }
-        }
-        __syncwarp();
-    } else if (warp == 1) {
-        if (lane == 0) {
-            for (int i = 0; i < nkb; ++i) {
-                const int st = i % NST;
-                mbar_wait(full0 + 8 * st, (i / NST) & 1);
-                tc_fence_after();
-                const uint32_t sa = smem_u32(smem + st * STAGE), sb = sa + S * 2 * OZ_BLK;
-#pragma unroll
-                for (int kk = 0; kk < OZ_BK / 32; ++kk) {
-#pragma unroll
-                    for (int s = 0; s < S; ++s) {
-                        const uint64_t da = umma_desc_sw64(sa + s * 2 * OZ_BLK + kk * 32);
-#pragma unroll
-                        for (int t = 0; t + s < S; ++t) {
-                            const uint64_t db = umma_desc_sw64(sb + t * OZ_BLK + kk * 32);
-                            tc_mma_i8(tmem + (uint32_t)((s + t) * OZ_BN), da, db, OZ_IDESC, (i | kk | s) != 0);
-                        }
-                    }
-                }
-                tc_commit(empty0 + 8 * st);
-            }
-            tc_commit(tfull);
-        }
-        __syncwarp();
-    } else {
-        const int q = warp & 3;
-        const int row = 32 * q + lane;
-        const int gr = ti * OZ_BM + row;
-        if (nkb > 0) {
-            mbar_wait(tfull, 0);
-            tc_fence_after();
-        }
+    // the phase epilogue of one 16-column chunk of tile row `row`
+    const auto epi = [&](int row, int c, double(&acc)[16]) {
+        const int Mp = R.Mp, Wp = R.Wp, M = R.M;
+        const int gr = ti * OZ_BM + row, gc0 = tj * OZ_BN + 16 * c;
+        if (gr >= Mp || gc0 >= Mp) return;                  // outside the allocated matrix (128-row tiles overhang)
         const Layout lay = make_layout(R.Mp, R.Np, R.Wp, prm.D);
         double* base = ws + R.base;
-        const int Mp = R.Mp, Wp = R.Wp, M = R.M;
-        const double sa = gr < M ? oz_pow2(oz_scale(ws, R, S, abuf)[gr]) : 0.0;
-        const double* sbv = oz_scale(ws, R, S, bbuf);
-#pragma unroll 1
-        for (int c = 0; c < OZ_BN / 16; ++c) {
-            double acc[16];
+        const double sa = gr < M ? oz_pow2(oz_scale(ws, R, abuf)[gr]) : 0.0;
+        const double* sbv = oz_scale(ws, R, bbuf);
 #pragma unroll
-            for (int j = 0; j < 16; ++j) acc[j] = 0.0;
-            if (nkb > 0) {
-                // the S accumulators in two batches (register budget), smallest weights first
+        for (int j = 0; j < 16; ++j) acc[j] = (gc0 + j < M) ? acc[j] * sa * oz_pow2(sbv[gc0 + j]) : 0.0;
+        if (PH == PH_A || PH == PH_B) {
+            double* out = base + (PH == PH_A ? lay.A : lay.Bm) + (size_t)gr * Wp + gc0;
 #pragma unroll
-                for (int h = (S - 1) / 4; h >= 0; --h) {
-                    int32_t v[4][16];
+            for (int j = 0; j < 16; j += 2) *reinterpret_cast<double2*>(out + j) = make_double2(acc[j], acc[j + 1]);
+        } else if (PH == PH_GA) {        // G_A = m g_mu^T + 2 (T B - A) diag(g_v)
+            const double2* Am = reinterpret_cast<const double2*>(base + lay.A + (size_t)gr * Wp + gc0);
+            const double mi = base[lay.m + gr];
+            const double2* gmu = reinterpret_cast<const double2*>(base + lay.gmu + gc0);
+            const double2* gv = reinterpret_cast<const double2*>(base + lay.gv + gc0);
+            double2* out = reinterpret_cast<double2*>(base + lay.GA + (size_t)gr * Mp + gc0);
 #pragma unroll
-                    for (int g = 0; g < 4; ++g)
-                        if (4 * h + g < S)
-                            tc_ld16(tmem + ((uint32_t)(32 * q) << 16) + (uint32_t)((4 * h + g) * OZ_BN + 16 * c), v[g]);
-                    tc_wait_ld();
+            for (int j = 0; j < 8; ++j) {
+                const double2 a = Am[j], u = gmu[j], w = gv[j];
+                out[j] = make_double2(mi * u.x + 2.0 * w.x * (acc[2 * j] - a.x), mi * u.y + 2.0 * w.y * (acc[2 * j + 1] - a.y));
+            }
+        } else if (PH == PH_GT) {        // dT = tril(2 A diag(g_v) B^T + (T - diag(1/T_ii))/N), Adam on T
+            const double invN = 1.0 / (double)M;
+            if (gr < M) {
 #pragma unroll
-                    for (int g = 3; g >= 0; --g) {
-                        if (4 * h + g < S) {
-                            const double w = __longlong_as_double((long long)(1023 - (12 + 7 * (4 * h + g))) << 52);   // 2^-(12+7g)
-#pragma unroll
-                            for (int j = 0; j < 16; ++j) acc[j] = fma((double)v[g][j], w, acc[j]);
-                        }
+                for (int j = 0; j < 16; j += 2) {
+                    const int cc = gc0 + j;
+                    const size_t idx = (size_t)gr * Mp + cc;
+                    if (cc + 1 <= gr) {          // both elements in the lower triangle: 128-bit loads / stores
+                        double2 p = *reinterpret_cast<const double2*>(base + lay.T + idx);
+                        double2 m1 = *reinterpret_cast<const double2*>(base + lay.Tm + idx);
+                        double2 m2 = *reinterpret_cast<const double2*>(base + lay.Tv + idx);
+                        const double ga = 2.0 * acc[j] + p.x * invN;
+                        const double gb = 2.0 * acc[j + 1] + (p.y - (cc + 1 == gr ? 1.0 / p.y : 0.0)) * invN;
+                        adam_update(p.x, m1.x, m2.x, ga, prm);
+                        adam_update(p.y, m1.y, m2.y, gb, prm);
+                        *reinterpret_cast<double2*>(base + lay.T + idx) = p;
+                        *reinterpret_cast<double2*>(base + lay.Tm + idx) = m1;
+                        *reinterpret_cast<double2*>(base + lay.Tv + idx) = m2;
+                    } else if (cc == gr) {       // the diagonal element alone
+                        double p = base[lay.T + idx];
+                        const double g = 2.0 * acc[j] + (p - 1.0 / p) * invN;
+                        double m1 = base[lay.Tm + idx], m2 = base[lay.Tv + idx];
+                        adam_update(p, m1, m2, g, prm);
+                        base[lay.T + idx] = p;
+                        base[lay.Tm + idx] = m1;
+                        base[lay.Tv + idx] = m2;
                     }
                 }
             }
-            const int gc0 = tj * OZ_BN + 16 * c;
-            if (gr >= Mp || gc0 >= Mp) continue;                // outside the allocated matrix (128-row tiles overhang)
+        } else if (PH == PH_GC || PH == PH_Y) {
+            double* out = base + (PH == PH_GC ? lay.GC : lay.GA) + (size_t)gr * Mp + gc0;
 #pragma unroll
-            for (int j = 0; j < 16; ++j) acc[j] = (gc0 + j < M) ? acc[j] * sa * oz_pow2(sbv[gc0 + j]) : 0.0;
-            if (PH == PH_A || PH == PH_B) {
-                double* out = base + (PH == PH_A ? lay.A : lay.Bm) + (size_t)gr * Wp + gc0;
+            for (int j = 0; j < 16; j += 2) *reinterpret_cast<double2*>(out + j) = make_double2(acc[j], acc[j + 1]);
+        } else if (PH == PH_GL) {        // S = -sym(Phi(G_A A^T)) mirrored, into the B buffer
+            double* out = base + lay.Bm;
 #pragma unroll
-                for (int j = 0; j < 16; j += 2) *reinterpret_cast<double2*>(out + j) = make_double2(acc[j], acc[j + 1]);
-            } else if (PH == PH_GA) {        // G_A = m g_mu^T + 2 (T B - A) diag(g_v)
-                const double2* Am = reinterpret_cast<const double2*>(base + lay.A + (size_t)gr * Wp + gc0);
-                const double mi = base[lay.m + gr];
-                const double2* gmu = reinterpret_cast<const double2*>(base + lay.gmu + gc0);
-                const double2* gv = reinterpret_cast<const double2*>(base + lay.gv + gc0);
-                double2* out = reinterpret_cast<double2*>(base + lay.GA + (size_t)gr * Mp + gc0);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const double2 a = Am[j], u = gmu[j], w = gv[j];
-                    out[j] = make_double2(mi * u.x + 2.0 * w.x * (acc[2 * j] - a.x), mi * u.y + 2.0 * w.y * (acc[2 * j + 1] - a.y));
+            for (int j = 0; j < 16; ++j) {
+                const int cc = gc0 + j;
+                const double val = -0.5 * acc[j];
+                if (cc <= gr) {
+                    out[(size_t)gr * Wp + cc] = val;
+                    if (cc < gr) out[(size_t)cc * Wp + gr] = val;
                 }
-            } else if (PH == PH_GT) {        // dT = tril(2 A diag(g_v) B^T + (T - diag(1/T_ii))/N), Adam on T
-                const double invN = 1.0 / (double)M;
-                if (gr < M) {
+            }
+        } else if (PH == PH_GK) {        // G_K = L^-T Y, symmetric: lower part + mirror, into the B buffer
+            double* out = base + lay.Bm;
 #pragma unroll
-                    for (int j = 0; j < 16; j += 2) {
-                        const int cc = gc0 + j;
-                        const size_t idx = (size_t)gr * Mp + cc;
-                        if (cc + 1 <= gr) {          // both elements in the lower triangle: 128-bit loads / stores
-                            double2 p = *reinterpret_cast<const double2*>(base + lay.T + idx);
-                            double2 m1 = *reinterpret_cast<const double2*>(base + lay.Tm + idx);
-                            double2 m2 = *reinterpret_cast<const double2*>(base + lay.Tv + idx);
-                            const double ga = 2.0 * acc[j] + p.x * invN;
-                            const double gb = 2.0 * acc[j + 1] + (p.y - (cc + 1 == gr ? 1.0 / p.y : 0.0)) * invN;
-                            adam_update(p.x, m1.x, m2.x, ga, prm);
-                            adam_update(p.y, m1.y, m2.y, gb, prm);
-                            *reinterpret_cast<double2*>(base + lay.T + idx) = p;
-                            *reinterpret_cast<double2*>(base + lay.Tm + idx) = m1;
-                            *reinterpret_cast<double2*>(base + lay.Tv + idx) = m2;
-                        } else if (cc == gr) {       // the diagonal element alone
-                            double p = base[lay.T + idx];
-                            const double g = 2.0 * acc[j] + (p - 1.0 / p) * invN;
-                            double m1 = base[lay.Tm + idx], m2 = base[lay.Tv + idx];
-                            adam_update(p, m1, m2, g, prm);
-                            base[lay.T + idx] = p;
-                            base[lay.Tm + idx] = m1;
-                            base[lay.Tv + idx] = m2;
-                        }
-                    }
-                }
-            } else if (PH == PH_GC || PH == PH_Y) {
-                double* out = base + (PH == PH_GC ? lay.GC : lay.GA) + (size_t)gr * Mp + gc0;
-#pragma unroll
-                for (int j = 0; j < 16; j += 2) *reinterpret_cast<double2*>(out + j) = make_double2(acc[j], acc[j + 1]);
-            } else if (PH == PH_GL) {        // S = -sym(Phi(G_A A^T)) mirrored, into the B buffer
-                double* out = base + lay.Bm;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    const int cc = gc0 + j;
-                    const double val = -0.5 * acc[j];
-                    if (cc <= gr) {
-                        out[(size_t)gr * Wp + cc] = val;
-                        if (cc < gr) out[(size_t)cc * Wp + gr] = val;
-                    }
-                }
-            } else if (PH == PH_GK) {        // G_K = L^-T Y, symmetric: lower part + mirror, into the B buffer
-                double* out = base + lay.Bm;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    const int cc = gc0 + j;
-                    if (cc <= gr) {
-                        out[(size_t)gr * Wp + cc] = acc[j];
-                        if (cc < gr) out[(size_t)cc * Wp + gr] = acc[j];
-                    }
+            for (int j = 0; j < 16; ++j) {
+                const int cc = gc0 + j;
+                if (cc <= gr) {
+                    out[(size_t)gr * Wp + cc] = acc[j];
+                    if (cc < gr) out[(size_t)cc * Wp + gr] = acc[j];
                 }
             }
         }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        __syncwarp();
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
-    }
+    };
+    const size_t kstride = (size_t)oz_rb(R.Mp) * OZ_BLK, plane = oz_plane_bytes(R.Mp);
+    oz_tile<OZ_S>(oz_smem_b, oz_buf(ws, R, abuf) + k0 * kstride + (size_t)2 * ti * OZ_BLK, kstride, plane,
+                  oz_buf(ws, R, bbuf) + k0 * kstride + (size_t)tj * OZ_BLK, kstride, plane, k1 - k0, epi);
 }

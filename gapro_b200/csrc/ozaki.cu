@@ -12,14 +12,9 @@
 //   Error: <= (S+1) 2^-(7S) of the row-max x row-max x K bound (1.6e-12 at S = 6), i.e. normwise like a float64
 //   GEMM with a ~1e4 larger unit roundoff; S(S+1)/2 = 21 int8 products per float64 product at S = 6.
 //
-// Kernel k_oz_gemm: one CTA per 128 x 64 output tile, warp-specialised -
-//   warp 0    producer: per 64-deep k-block ONE mbarrier transaction of S x (8 KB + 4 KB) `cp.async.bulk` copies
-//             (the digit planes are stored in global memory block by block ALREADY in the 64-byte-swizzled K-major
-//             shared-memory layout the UMMA descriptors describe, so a plain bulk copy lands them ready to use);
-//   warp 1    one elected thread issues tcgen05.mma.cta_group::1.kind::i8 (M = 128, N = 64, K = 32) for all pairs
-//             of the k-block into S TMEM accumulators (S x 64 columns), tcgen05.commit releases the stage;
-//   warps 2-5 epilogue: tcgen05.ld the S accumulators of their 32 TMEM lanes, float64 recombination, scaling, store.
-// Three 72 KB stages (216 KB of shared memory), 512 TMEM columns allocated, one CTA per SM.
+// Kernel k_oz_gemm: one CTA per 128 x 64 output tile, the warp-specialised main loop oz_tile (ozaki_ptx.cuh) with an
+// epilogue that scales and stores.  oz_stages(S) stages of S x 12 KB: three of 72 KB (216 KB of shared memory) at
+// S = 6, two of 96 KB (192 KB) at S = 8; 512 TMEM columns allocated, one CTA per SM.
 #include <vector>
 
 #include "common.cuh"
@@ -44,127 +39,19 @@ struct OzGemm {
 template <int S>
 __global__ void __launch_bounds__(OZ_THREADS, 1) k_oz_gemm(OzGemm P) {
     extern __shared__ __align__(1024) uint8_t oz_smem[];
-    constexpr int STAGE = oz_stage_bytes(S);
-    constexpr int OZ_STAGES = oz_stages(S);
-    uint8_t* smem = (uint8_t*)(((uintptr_t)oz_smem + 1023) & ~(uintptr_t)1023);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + OZ_STAGES * STAGE);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * OZ_STAGES + 1);
-    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + OZ_STAGES), tfull = smem_u32(bars + 2 * OZ_STAGES);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int ti = blockIdx.x / P.tiles_n, tj = blockIdx.x % P.tiles_n;
-    const int nkb = P.kb_total;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < OZ_STAGES; ++s) {
-            mbar_init(full0 + 8 * s, 1);
-            mbar_init(empty0 + 8 * s, 1);
-        }
-        mbar_init(tfull, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            const size_t a_plane = (size_t)P.kb_total * P.a_rb * OZ_BLK, b_plane = (size_t)P.kb_total * P.b_rb * OZ_BLK;
-            for (int i = 0; i < nkb; ++i) {
-                const int st = i % OZ_STAGES;
-                mbar_wait(empty0 + 8 * st, ((i / OZ_STAGES) & 1) ^ 1);
-                mbar_expect_tx(full0 + 8 * st, (uint32_t)STAGE);
-                const uint32_t dst = smem_u32(smem + st * STAGE);
-                const uint8_t* ga = P.a + ((size_t)i * P.a_rb + 2 * ti) * OZ_BLK;
-                const uint8_t* gb = P.b + ((size_t)i * P.b_rb + tj) * OZ_BLK;
+    const auto epi = [&](int row, int c, const double(&acc)[16]) {
+        const int gr = ti * OZ_BM + row, gc0 = tj * OZ_BN + 16 * c;
+        if (gr >= P.M) return;
+        const double sa = P.sa[gr];
+        double* out = P.C + (size_t)gr * P.ldc + gc0;
 #pragma unroll
-                for (int s = 0; s < S; ++s) {
-                    bulk_g2s(dst + s * 2 * OZ_BLK, ga + s * a_plane, 2 * OZ_BLK, full0 + 8 * st);
-                    bulk_g2s(dst + S * 2 * OZ_BLK + s * OZ_BLK, gb + s * b_plane, OZ_BLK, full0 + 8 * st);
-                }
-            }
-        }
-        __syncwarp();
-    } else if (warp == 1) {
-        if (lane == 0) {
-            for (int i = 0; i < nkb; ++i) {
-                const int st = i % OZ_STAGES;
-                mbar_wait(full0 + 8 * st, (i / OZ_STAGES) & 1);
-                tc_fence_after();
-                const uint32_t sa = smem_u32(smem + st * STAGE), sb = sa + S * 2 * OZ_BLK;
-#pragma unroll
-                for (int kk = 0; kk < OZ_BK / 32; ++kk) {
-#pragma unroll
-                    for (int s = 0; s < S; ++s) {
-                        const uint64_t da = umma_desc_sw64(sa + s * 2 * OZ_BLK + kk * 32);
-#pragma unroll
-                        for (int t = 0; t + s < S; ++t) {
-                            const uint64_t db = umma_desc_sw64(sb + t * OZ_BLK + kk * 32);
-                            tc_mma_i8(tmem + (uint32_t)((s + t) * OZ_BN), da, db, OZ_IDESC, (i | kk | s) != 0);
-                        }
-                    }
-                }
-                tc_commit(empty0 + 8 * st);      // frees the stage when these MMAs have read it
-            }
-            tc_commit(tfull);                    // accumulators complete
-        }
-        __syncwarp();
-    } else {
-        // epilogue warps 2..5: TMEM lane quarter = warp % 4
-        const int q = warp & 3;
-        const int row = 32 * q + lane;
-        const int gr = ti * OZ_BM + row;
-        if (nkb > 0) {
-            mbar_wait(tfull, 0);
-            tc_fence_after();
-        }
-        const double sa = gr < P.M ? P.sa[gr] : 0.0;
-#pragma unroll 1
-        for (int c = 0; c < OZ_BN / 16; ++c) {
-            double acc[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) acc[j] = 0.0;
-            if (nkb > 0) {
-                // the S accumulators in two batches (register budget), smallest weights first
-#pragma unroll
-                for (int h = (S - 1) / 4; h >= 0; --h) {
-                    int32_t v[4][16];
-#pragma unroll
-                    for (int g = 0; g < 4; ++g)
-                        if (4 * h + g < S)
-                            tc_ld16(tmem + ((uint32_t)(32 * q) << 16) + (uint32_t)((4 * h + g) * OZ_BN + 16 * c), v[g]);
-                    tc_wait_ld();
-#pragma unroll
-                    for (int g = 3; g >= 0; --g) {
-                        if (4 * h + g < S) {
-                            const double w = __longlong_as_double((long long)(1023 - (12 + 7 * (4 * h + g))) << 52);   // 2^-(12+7g)
-#pragma unroll
-                            for (int j = 0; j < 16; ++j) acc[j] = fma((double)v[g][j], w, acc[j]);
-                        }
-                    }
-                }
-            }
-            if (gr < P.M) {
-                const int gc0 = tj * OZ_BN + 16 * c;
-                double* out = P.C + (size_t)gr * P.ldc + gc0;
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                    if (gc0 + j < P.N) out[j] = acc[j] * sa * P.sb[gc0 + j];
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        __syncwarp();
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
-    }
+        for (int j = 0; j < 16; ++j)
+            if (gc0 + j < P.N) out[j] = acc[j] * sa * P.sb[gc0 + j];
+    };
+    const size_t a_kstride = (size_t)P.a_rb * OZ_BLK, b_kstride = (size_t)P.b_rb * OZ_BLK;
+    oz_tile<S>(oz_smem, P.a + (size_t)2 * ti * OZ_BLK, a_kstride, P.kb_total * a_kstride, P.b + (size_t)tj * OZ_BLK,
+               b_kstride, P.kb_total * b_kstride, P.kb_total, epi);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -201,32 +88,10 @@ template <int S>
 __global__ void __launch_bounds__(256)
 k_oz_slice(const double* __restrict__ X, int ld, int nvec, int K, int trans, const double* __restrict__ ks,
            const double* __restrict__ scale, uint8_t* __restrict__ planes, int rb_total, int kb_total) {
-    constexpr int LD = 68;                         // + k/16 skew: conflict-free 16-double reads per (vector, chunk)
-    __shared__ double blk[64 * LD + 8];
-    const int kb = blockIdx.x, rb = blockIdx.y;
-    const int v0 = rb * 64, k0 = kb * 64;
-    // stage the 64 x 64 source block (zero outside the matrix)
-    for (int e = threadIdx.x; e < 64 * 64; e += 256) {
-        const int a = e >> 6, b = e & 63;          // b runs along the contiguous direction of X
-        const int v = trans ? b : a, k = trans ? a : b;
-        double x = 0.0;
-        if (v0 + v < nvec && k0 + k < K) {
-            x = trans ? X[(size_t)(k0 + k) * ld + v0 + v] : X[(size_t)(v0 + v) * ld + k0 + k];
-            if (ks) x *= ks[k0 + k];
-        }
-        blk[v * LD + k + (k >> 4)] = x;
-    }
-    __syncthreads();
-    const int t = threadIdx.x;
-    const int atom = t >> 5, r = (t & 31) >> 2, c = t & 3;
-    const int v = 8 * atom + r;
-    const double inv = (v0 + v < nvec) ? 1.0 / scale[v0 + v] : 0.0;      // exact: a power of two
-    double y[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) y[j] = blk[v * LD + 16 * c + j + c] * inv * 64.0;      // |y| < 64
-    const size_t plane = (size_t)kb_total * rb_total * OZ_BLK;
-    uint8_t* dst = planes + ((size_t)kb * rb_total + rb) * OZ_BLK + atom * 512 + r * 64 + ((c ^ ((r >> 1) & 3)) * 16);
-    emit_digits<S>(y, dst, plane);
+    oz_slice_block<S>(
+        X, ld, trans, ks, blockIdx.x, blockIdx.y, [&](int v, int k) { return v < nvec && k < K; },
+        [&](int v) { return v < nvec ? 1.0 / scale[v] : 0.0; }, 64.0,      // exact: a power of two
+        planes, kb_total, rb_total);
 }
 
 struct OzWs {

@@ -320,7 +320,7 @@ int gapro_occupancy_points(const double* xyz, const int32_t* spp_gid, const int3
  * Float64 products on tcgen05 by int8 digit planes ("Ozaki scheme"; csrc/ozaki.cu).  C[M,N] = op(A) op(B)^T:
  * trans = 0 - the operand is stored [vectors, K] row-major, trans = 1 - [K, vectors] row-major; kscale (optional,
  * dev double[K]) multiplies the A operand along k (A diag(kscale) B^T, the dT product of the GP step).  S digits per
- * operand (2..7; 6 gives ~1e-12 of the row-norm bound), S(S+1)/2 int8 products.  ws 1024-byte aligned.  The last of
+ * operand (2..8; 6 gives ~1e-12 of the row-norm bound), S(S+1)/2 int8 products.  ws 1024-byte aligned.  The last of
  * `reps` runs is timed with CUDA events: ms_slice (scaling + digit planes), ms_gemm (the tcgen05 kernel).
  */
 size_t gapro_ozaki_workspace_bytes(int32_t M, int32_t N, int32_t K, int32_t S);

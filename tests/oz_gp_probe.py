@@ -1,5 +1,5 @@
-"""Development probe (GPU): accuracy and time of whole GP fits with the tcgen05 digit-plane path against the golden
-fp64-oracle vectors, for several digit counts / thresholds.  Env knobs are read per call by the library."""
+"""Development probe (GPU): accuracy and time of whole GP fits on the DMMA path and on the tcgen05 digit-plane path
+(8 digits) against the golden fp64-oracle vectors.  Env knobs are read per call by the library."""
 import os
 import sys
 import time
@@ -21,10 +21,7 @@ def run(case_id, M, D, N, mu_ref, var_ref, label):
     dev = torch.device("cuda:0")
     X, n1, Xt, noise = gp_case(case_id, M, D, N)
     feats = torch.from_numpy(np.concatenate([X, Xt])).to(dev)
-    for env in ({"GAPRO_GP_OZAKI": "0"}, {"GAPRO_GP_OZAKI": "1", "GAPRO_GP_OZAKI_S": "6"},
-                {"GAPRO_GP_OZAKI": "1", "GAPRO_GP_OZAKI_S": "7"}, {"GAPRO_GP_OZAKI": "1", "GAPRO_GP_OZAKI_S": "8"}):
-        for k in ("GAPRO_GP_OZAKI", "GAPRO_GP_OZAKI_S", "GAPRO_GP_OZAKI_MIN_M"):
-            os.environ.pop(k, None)
+    for env in ({"GAPRO_GP_OZAKI": "0"}, {"GAPRO_GP_OZAKI": "1"}):
         os.environ.update(env)
         os.environ["GAPRO_GP_OZAKI_MIN_M"] = "512"
         ts = []

@@ -14,10 +14,9 @@ from tests.golden.make_golden import gp_case  # noqa: E402
 PH = _debug.PHASES
 
 
-def state(case, iters, stop, oz, S="7"):
+def state(case, iters, stop, oz):
     os.environ["GAPRO_GP_OZAKI"] = "1" if oz else "0"
     os.environ["GAPRO_GP_OZAKI_MIN_M"] = "128"
-    os.environ["GAPRO_GP_OZAKI_S"] = S
     X, n1, Xt, noise = case
     dev = torch.device("cuda:0")
     feats = torch.from_numpy(np.concatenate([X, Xt])).to(dev)
