@@ -33,6 +33,8 @@ _SIGNATURES = {
                                               c_float, P, P, P]),
     "gapro_multibox_workspace_bytes": (c_size_t, [c_int64]),
     "gapro_multibox_sources": (ctypes.c_int, [P, P, P, P, c_int32, c_int64, P, P, c_size_t, P]),
+    "gapro_heuristic_finalize": (ctypes.c_int, [P, P, P, P, P, P, c_int32, c_int32, c_int32, c_int64, c_int32, P, P,
+                                                P, P]),
     "gapro_pool_feats": (ctypes.c_int, [P, P, P, c_int32, c_int32, P, P]),
     "gapro_enumerate_events": (ctypes.c_int, [P, c_int32, P, P, c_int32, P, P, P, c_int32]),
     "gapro_box_iou": (ctypes.c_int, [P, c_int32, P]),

@@ -773,6 +773,69 @@ extern "C" int gapro_heuristic_labels(const double* xyz, const int32_t* perm, co
 }
 
 // =============================================================================================
+// Heuristic labels -> final labels (gen_ps_utils.py:283-288 / :559-564).  Scene-local box index b >= 0:
+// sem = cls[box_off[scene] + b], inst = b; -1 (background): sem = instance_classes, inst = -100; -2 (undecided
+// under rule "none", per point only): sem = inst = -100.  Superpoint-aligned results become the 16-byte records
+// (sem, inst, 1.0f, 0) of k_broadcast; per-point results are written directly.  One thread per element.
+// =============================================================================================
+__device__ __forceinline__ int2 heuristic_final(int b, int sc, const int32_t* __restrict__ box_off,
+                                                const int64_t* __restrict__ cls, int instance_classes) {
+    if (b >= 0) return make_int2((int32_t)cls[box_off[sc] + b], b);
+    return make_int2(b == -1 ? instance_classes : -100, -100);
+}
+
+__global__ void __launch_bounds__(256)
+k_heuristic_final_spp(const int32_t* __restrict__ inst_spp, const int32_t* __restrict__ spp_off,
+                      const int32_t* __restrict__ box_off, const int64_t* __restrict__ cls, int instance_classes,
+                      int n_scenes, int s_total, int4* __restrict__ packed_spp) {
+    const int g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= s_total) return;
+    const int b = inst_spp[g];
+    const int2 r = heuristic_final(b, b >= 0 ? gapro_find_segment(spp_off, n_scenes, g) : 0, box_off, cls,
+                                   instance_classes);
+    packed_spp[g] = make_int4(r.x, r.y, __float_as_int(1.0f), 0);
+}
+
+__global__ void __launch_bounds__(256)
+k_heuristic_final_pt(const int32_t* __restrict__ inst_pt, const int64_t* __restrict__ pt_off,
+                     const int32_t* __restrict__ box_off, const int64_t* __restrict__ cls, int instance_classes,
+                     int n_scenes, int64_t n, int32_t* __restrict__ sem, int32_t* __restrict__ inst) {
+    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    const int b = inst_pt[p];
+    const int2 r = heuristic_final(b, b >= 0 ? find_scene_pt(pt_off, n_scenes, p) : 0, box_off, cls, instance_classes);
+    sem[p] = r.x;
+    inst[p] = r.y;
+}
+
+extern "C" int gapro_heuristic_finalize(const int32_t* inst_spp, const int32_t* inst_pt, const int32_t* spp_off_dev,
+                                        const int64_t* pt_off_dev, const int32_t* box_off_dev,
+                                        const int64_t* boxes_cls, int32_t instance_classes, int32_t n_scenes,
+                                        int32_t s_total, int64_t n_points, int32_t spp_align, void* packed_spp,
+                                        int32_t* sem, int32_t* inst, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GAPRO_REQUIRE(box_off_dev && boxes_cls, "gapro_heuristic_finalize: null pointer");
+    GAPRO_REQUIRE(n_scenes > 0, "gapro_heuristic_finalize: n_scenes must be positive");
+    const int T = 256;
+    if (spp_align) {
+        GAPRO_REQUIRE(inst_spp && spp_off_dev, "gapro_heuristic_finalize: null pointer");
+        GAPRO_REQUIRE(packed_spp, "gapro_heuristic_finalize: missing output array (packed_spp)");
+        GAPRO_REQUIRE(s_total > 0, "gapro_heuristic_finalize: empty batch");
+        GAPRO_REQUIRE((uintptr_t)packed_spp % 16 == 0, "gapro_heuristic_finalize: packed_spp must be 16-byte aligned");
+        k_heuristic_final_spp<<<(unsigned)((s_total + T - 1) / T), T, 0, stream>>>(
+            inst_spp, spp_off_dev, box_off_dev, boxes_cls, instance_classes, n_scenes, s_total, (int4*)packed_spp);
+    } else {
+        GAPRO_REQUIRE(inst_pt && pt_off_dev, "gapro_heuristic_finalize: null pointer");
+        GAPRO_REQUIRE(sem && inst, "gapro_heuristic_finalize: missing output array (sem, inst)");
+        GAPRO_REQUIRE(n_points > 0, "gapro_heuristic_finalize: empty batch");
+        k_heuristic_final_pt<<<(unsigned)((n_points + T - 1) / T), T, 0, stream>>>(
+            inst_pt, pt_off_dev, box_off_dev, boxes_cls, instance_classes, n_scenes, n_points, sem, inst);
+    }
+    GAPRO_KERNEL_CHECK();
+    return GAPRO_OK;
+}
+
+// =============================================================================================
 // B — feature pooling (gen_ps_utils.py:357): float32 sum in point-index order, / float32 count
 // =============================================================================================
 // One warp per superpoint.  For every chunk of 32 points the warp loads the point indices with one

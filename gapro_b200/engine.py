@@ -386,76 +386,78 @@ class GaproEngine:
         return out, dbg
 
     # ------------------------------------------------------------------ heuristic labelers (SURVEY 8f)
-    def run_heuristic(self, coords_float, spp, instance_cls, instance_box, instance_box_volume, instance_classes=18,
-                      rule="volume", spp_align=True, occ_thresh=None):
-        """One scene through the heuristic labelers: per-point containment in the instance boxes, the rule
-        for points in several boxes, optional majority vote per superpoint.  Returns (sem[N] i32, inst[N] i32)."""
+    def run_heuristic(self, scenes: Sequence[SceneInputs], rule="volume", spp_align=True, occ_thresh=None,
+                      instance_classes=18):
+        """Scenes through the heuristic labelers in one pass: per-point containment in the instance boxes, the rule
+        for points in several boxes, optional majority vote per superpoint, final labels.  Only the coordinates, the
+        superpoints and the instance boxes / classes / volumes of each scene are read (no wall boxes, no floor slab).
+        Returns one (sem[N] i32, inst[N] i32) pair of device views per scene."""
         lib, dev = self.lib, self.device
         stream = torch.cuda.current_stream(dev).cuda_stream
-        xyz = coords_float.to(dev, torch.float64).contiguous()
-        N = int(xyz.shape[0])
-        K = int(instance_box.shape[0])
+        ns = len(scenes)
+        if ns == 0:
+            return []
+        rule_id = {"volume": 0, "dist": 1, "none": 2}[rule]
+        n_pts = [int(s.coords_float.shape[0]) for s in scenes]
+        pt_off = np.zeros(ns + 1, dtype=np.int64)
+        pt_off[1:] = np.cumsum(n_pts)
+        N = int(pt_off[-1])
+        n_box = np.array([int(s.instance_box.shape[0]) for s in scenes], dtype=np.int32)
+        box_off = np.zeros(ns + 1, dtype=np.int32)
+        box_off[1:] = np.cumsum(n_box)
         words = 1
-        while 32 * words < K:
+        while 32 * words < int(n_box.max()):
             words *= 2
         if words > 8:
             raise ValueError("more than 256 boxes in one scene")
-        boxes = instance_box.to(dev).float().contiguous()
-        vol = instance_box_volume.to(dev).float().contiguous()
-        cls = instance_cls.to(dev, torch.int64)
-        pt_off = np.array([0, N], dtype=np.int64)
+        cat = (lambda ts: ts[0].contiguous()) if ns == 1 else (lambda ts: torch.cat(ts, 0))
+        xyz = cat([s.coords_float.to(dev, torch.float64) for s in scenes])
+        spp_raw = cat([s.spp.to(dev, torch.int64).reshape(-1) for s in scenes])
+        # the boxes stay float32 (gen_ps.py:80): margins and centres are float32 values in the kernels
+        boxes = cat([s.instance_box.to(dev).float().reshape(-1, 6) for s in scenes])
+        vol = cat([s.instance_box_volume.to(dev).float().reshape(-1) for s in scenes])
+        cls = cat([s.instance_cls.to(dev, torch.int64).reshape(-1) for s in scenes])
+
         spp_gid = torch.empty(N, dtype=torch.int32, device=dev)
         perm = torch.empty(N, dtype=torch.int32, device=dev)
         seg_off = torch.empty(N + 1, dtype=torch.int32, device=dev)
-        spp_off = np.zeros(2, dtype=np.int32)
-        ws = self._workspace("densify", lib.gapro_densify_workspace_bytes(N, 1))
-        spp_raw = spp.to(dev, torch.int64).reshape(-1).contiguous()
-        _lib.check(lib.gapro_densify_spp(spp_raw.data_ptr(), pt_off.ctypes.data, 1, spp_gid.data_ptr(), perm.data_ptr(),
+        spp_off = np.zeros(ns + 1, dtype=np.int32)
+        ws = self._workspace("densify", lib.gapro_densify_workspace_bytes(N, ns))
+        _lib.check(lib.gapro_densify_spp(spp_raw.data_ptr(), pt_off.ctypes.data, ns, spp_gid.data_ptr(), perm.data_ptr(),
                                          seg_off.data_ptr(), spp_off.ctypes.data, ws.data_ptr(), ws.numel(), stream),
                    "gapro_densify_spp")
         St = int(spp_off[-1])
-        spp_off_dev = self._dev(spp_off)
-        box_off_dev = self._dev(np.array([0, K], dtype=np.int32))
-        rule_id = {"volume": 0, "dist": 1, "none": 2}[rule]
-        inst_spp = torch.empty(St, dtype=torch.int32, device=dev)
-        inst_pt = torch.empty(N, dtype=torch.int32, device=dev)
+        offs = self._dev(np.concatenate([box_off, spp_off]))         # one upload for both int32 offset tables
+        box_off_dev, spp_off_dev = offs[:ns + 1], offs[ns + 1:]
+        pt_off_dev = self._dev(pt_off) if rule_id == 1 or not spp_align else None
         thr = -1.0 if occ_thresh is None else float(np.float32(occ_thresh))
         dist_src = None
         if rule_id == 1:
             # the reference measures the k-th multi-box point from the coordinates of point k (gen_ps_utils.py:516,526)
             dist_src = torch.empty(N, dtype=torch.int32, device=dev)
             mws = self._workspace("multibox", lib.gapro_multibox_workspace_bytes(N))
-            pt_off_dev = self._dev(pt_off)
             _lib.check(lib.gapro_multibox_sources(xyz.data_ptr(), pt_off_dev.data_ptr(), box_off_dev.data_ptr(),
-                                                  boxes.data_ptr(), 1, N, dist_src.data_ptr(), mws.data_ptr(),
+                                                  boxes.data_ptr(), ns, N, dist_src.data_ptr(), mws.data_ptr(),
                                                   mws.numel(), stream), "gapro_multibox_sources")
+        inst_spp = torch.empty(St, dtype=torch.int32, device=dev) if spp_align else None
+        inst_pt = None if spp_align else torch.empty(N, dtype=torch.int32, device=dev)
         _lib.check(lib.gapro_heuristic_labels(xyz.data_ptr(), perm.data_ptr(), seg_off.data_ptr(), spp_off_dev.data_ptr(),
-                                              box_off_dev.data_ptr(), boxes.data_ptr(), vol.data_ptr(),
-                                              0 if dist_src is None else dist_src.data_ptr(), 1, St, words,
-                                              rule_id, 1 if spp_align else 0, thr, inst_spp.data_ptr(),
-                                              inst_pt.data_ptr(), stream), "gapro_heuristic_labels")
+                                              box_off_dev.data_ptr(), boxes.data_ptr(), vol.data_ptr(), _ptr(dist_src),
+                                              ns, St, words, rule_id, 1 if spp_align else 0, thr, _ptr(inst_spp),
+                                              _ptr(inst_pt), stream), "gapro_heuristic_labels")
+        sem = torch.empty(N, dtype=torch.int32, device=dev)
+        inst = torch.empty(N, dtype=torch.int32, device=dev)
+        packed = torch.empty((St, 4), dtype=torch.int32, device=dev) if spp_align else None
+        _lib.check(lib.gapro_heuristic_finalize(_ptr(inst_spp), _ptr(inst_pt), spp_off_dev.data_ptr(), _ptr(pt_off_dev),
+                                                box_off_dev.data_ptr(), cls.data_ptr(), int(instance_classes), ns, St,
+                                                N, 1 if spp_align else 0, _ptr(packed), _ptr(None if spp_align else sem),
+                                                _ptr(None if spp_align else inst), stream), "gapro_heuristic_finalize")
         if spp_align:
-            # per-superpoint semantics (gen_ps_utils.py:283-288 / :559-564), then the 128-bit broadcast kernel
-            sem_spp = torch.full((St,), -100, dtype=torch.int32, device=dev)
-            pos = inst_spp >= 0
-            sem_spp[pos] = cls[inst_spp[pos].long()].int()
-            sem_spp[inst_spp == -1] = int(instance_classes)
-            inst_out = torch.where(pos, inst_spp, torch.full_like(inst_spp, -100))
-            packed = torch.stack([sem_spp, inst_out, torch.ones_like(sem_spp).float().view(torch.int32),
-                                  torch.zeros_like(sem_spp)], dim=1).contiguous()
-            sem = torch.empty(N, dtype=torch.int32, device=dev)
-            inst = torch.empty(N, dtype=torch.int32, device=dev)
+            # per-superpoint records (sem, inst, 1.0, 0) -> points with the 128-bit broadcast of the GP path
             prob = torch.empty(N, dtype=torch.float32, device=dev)
             _lib.check(lib.gapro_broadcast_labels(spp_gid.data_ptr(), N, packed.data_ptr(), sem.data_ptr(),
                                                   inst.data_ptr(), prob.data_ptr(), stream), "gapro_broadcast_labels")
-            return sem, inst
-        sem = torch.full((N,), -100, dtype=torch.int32, device=dev)
-        inst = torch.full((N,), -100, dtype=torch.int32, device=dev)
-        pos = inst_pt >= 0
-        sem[pos] = cls[inst_pt[pos].long()].int()
-        sem[inst_pt == -1] = int(instance_classes)
-        inst[pos] = inst_pt[pos]
-        return sem, inst
+        return [(sem[int(pt_off[i]):int(pt_off[i + 1])], inst[int(pt_off[i]):int(pt_off[i + 1])]) for i in range(ns)]
 
     def _make_noise(self, scenes, region_scene, region_m, total):
         """Standard-normal draws for the variational-mean init (gpytorch draws them from the unseeded

@@ -2,6 +2,7 @@
 /root/reference/gapro/gen_ps.py.
 
     python -m gapro_b200.gen_ps [--save_folder D] [--use_deepfeat] [--deepfeat_folder D] [--eval_pslabel]
+                                [--label_method {gp,box2mask,volume,dist,none}]
 
 keeps the reference flags (gen_ps.py:15-21), the relative dataset layout
 (dataset/scannetv2/{train,superpoints,scans_transform}), the output naming
@@ -9,7 +10,11 @@ keeps the reference flags (gen_ps.py:15-21), the relative dataset layout
 skip-if-exists resume rule (:39-41) and the saved tuple of five numpy arrays (:126-132).
 Additions: scenes are processed in batches on the GPU, and when launched under torchrun
 the sorted scene list is sharded across ranks (one process per GPU, no per-step collective;
-one final gather of per-scene metadata).
+one final gather of per-scene metadata).  --label_method other than gp writes the box-only
+heuristic labels instead (the alternative commented out at gen_ps.py:112-114:
+gen_pseudo_label_box2mask, or gen_pseudo_label with rule volume / dist / none), superpoint-aligned,
+in the same 5-tuple with prob = 1 and mu = var = -100; scenes are sharded round-robin, there is no
+GP cost pass.
 """
 from __future__ import annotations
 
@@ -24,7 +29,7 @@ import numpy as np
 import torch
 
 from .engine import SceneInputs
-from .gen_ps_utils import gen_pseudo_labels_batch, getInstanceInfo
+from .gen_ps_utils import gen_pseudo_labels_batch, gen_pseudo_labels_heuristic_batch, getInstanceInfo
 from .sharding import gather_records, shard_scenes
 
 DATA_ROOT = "dataset/scannetv2"
@@ -137,6 +142,15 @@ def save_pseudo_labels(path, result, per_point_uncertainty=False, spp_dense=None
     os.replace(tmp, path)
 
 
+def heuristic_result(sem, inst, spp):
+    """Heuristic labels as the 5-tuple the GP path saves: prob = 1 per point, mu = var = -100 (the reference's
+    "no GP value") per superpoint of the scene's raw superpoint ids `spp`."""
+    n_spp = int(torch.unique(spp).numel())
+    prob = torch.ones(sem.shape[0], dtype=torch.float32, device=sem.device)
+    none = torch.full((n_spp,), -100.0, dtype=torch.float32, device=sem.device)
+    return sem, inst, prob, none, none
+
+
 def _dist_env():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -187,7 +201,10 @@ def estimate_costs(items, args, device, pool):
     return costs
 
 
-def main(argv=None):
+LABEL_METHODS = ("gp", "box2mask", "volume", "dist", "none")
+
+
+def parse_args(argv=None):
     parser = argparse.ArgumentParser("GaPro_GenPS")
     parser.add_argument("--save_folder", type=str, default=osp.join(DATA_ROOT, "gaussian_process_kl_pseudo_labels"))
     parser.add_argument("--use_deepfeat", action="store_true")
@@ -208,7 +225,20 @@ def main(argv=None):
                              "instead of in the host loader threads; identical boxes")
     parser.add_argument("--balance", choices=["cost", "static"], default="cost",
                         help="multi-GPU sharding: LPT by a cost estimated from the cheap stages, or round-robin")
+    parser.add_argument("--label_method", choices=LABEL_METHODS, default="gp",
+                        help="gp: the GP labels of gen_ps.py; box2mask: gen_pseudo_label_box2mask; volume / dist / "
+                             "none: gen_pseudo_label with that heuristic rule (the alternative commented out at "
+                             "gen_ps.py:112-114).  The heuristic methods save prob = 1 and mu = var = -100")
     args = parser.parse_args(argv)
+    if args.label_method != "gp" and args.use_deepfeat:
+        parser.error(f"--use_deepfeat has no effect with --label_method {args.label_method}: "
+                     "the heuristic labelers read no features")
+    return args
+
+
+def main(argv=None):
+    args = parse_args(argv)
+    heuristic = args.label_method != "gp"
 
     rank, world, local = _dist_env()
     if world > 1:
@@ -234,7 +264,7 @@ def main(argv=None):
     pool = ThreadPoolExecutor(max_workers=max(1, min(args.load_workers, args.batch_scenes)))
     t0 = time.time()
     balance = None
-    if world > 1 and args.balance == "cost" and todo:
+    if world > 1 and args.balance == "cost" and todo and not heuristic:      # no GP work to balance otherwise
         from .sharding import balance_stats, lpt_assignment
         part = estimate_costs(todo[rank::world], args, device, pool)
         merged = {}
@@ -268,10 +298,15 @@ def main(argv=None):
             kept.append((scan, sem, inst))
         if not scenes:
             continue
-        results = gen_pseudo_labels_batch(scenes, instance_classes=18, ground_h=0.1, training_iter=50,
-                                          thresh_spp_occu=0.999, jitter_zz=args.jitter_zz, device=device,
-                                          on_error="mark")                          # gen_ps.py:106-110
-        errors = results.errors
+        if heuristic:
+            labels = gen_pseudo_labels_heuristic_batch(scenes, method=args.label_method, instance_classes=18,
+                                                       dataset_name="scannetv2", device=device)
+            results, errors = [heuristic_result(s, i, sc.spp) for (s, i), sc in zip(labels, scenes)], {}
+        else:
+            results = gen_pseudo_labels_batch(scenes, instance_classes=18, ground_h=0.1, training_iter=50,
+                                              thresh_spp_occu=0.999, jitter_zz=args.jitter_zz, device=device,
+                                              on_error="mark")                          # gen_ps.py:106-110
+            errors = results.errors
         for k, ((scan, sem, inst), res, sc) in enumerate(zip(kept, results, scenes)):
             if res is None:      # a GP region of this scene failed: the scene is reported, the others are saved
                 print(f"[rank {rank}] {scan}: not labelled - {errors.get(k)}", flush=True)

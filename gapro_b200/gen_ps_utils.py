@@ -1,4 +1,4 @@
-"""Host-side mirror of /root/reference/gapro/gen_ps_utils.py for the GP pseudo-label path.
+"""Host-side mirror of /root/reference/gapro/gen_ps_utils.py for the GP pseudo-label path and the heuristic labelers.
 
 Same call surface as the reference (names, argument meaning, return arity, dtypes,
 shapes — including the per-superpoint `mu`/`var` of gen_ps_utils.py:482), backed by the
@@ -14,7 +14,7 @@ from . import _lib
 from .engine import SceneInputs, get_engine
 
 __all__ = ["gen_pseudo_label_gaussian_process", "gen_pseudo_labels_batch", "gen_pseudo_label_box2mask",
-           "gen_pseudo_label", "getInstanceInfo", "getInstanceInfo_cuda", "batch_giou_cross", "is_box1_in_box2", "is_within_bb_torch",
+           "gen_pseudo_label", "gen_pseudo_labels_heuristic_batch", "getInstanceInfo", "getInstanceInfo_cuda", "batch_giou_cross", "is_box1_in_box2", "is_within_bb_torch",
            "SceneInputs"]
 
 
@@ -83,10 +83,8 @@ def gen_pseudo_label_box2mask(coords_float, spp, instance_cls, instance_box, ins
     """Drop-in for gen_pseudo_label_box2mask (/root/reference/gapro/gen_ps_utils.py:242-290): points in
     several boxes take the smallest one; for scannetv2 the labels are then aligned to superpoints by
     majority vote (spp_align_label, :99-129).  Returns (ps_semantic_label[N] int32, ps_instance_label[N] int32)."""
-    eng = get_engine(coords_float.device if coords_float.is_cuda else None)
-    return eng.run_heuristic(coords_float, spp, instance_cls, instance_box, instance_box_volume,
-                             instance_classes=instance_classes, rule="volume",
-                             spp_align=(dataset_name == "scannetv2"), occ_thresh=None)
+    return _heuristic_one(coords_float, spp, instance_cls, instance_box, instance_box_volume, "box2mask",
+                          instance_classes, dataset_name)
 
 
 def gen_pseudo_label(coords_float, spp, instance_cls, instance_box, instance_box_volume, instance_classes=18,
@@ -96,10 +94,36 @@ def gen_pseudo_label(coords_float, spp, instance_cls, instance_box, instance_box
     win if it holds at least 70 % of the superpoint (:538-550)."""
     if heuristic_rule not in ("volume", "dist", "none"):
         raise Exception
-    eng = get_engine(coords_float.device if coords_float.is_cuda else None)
-    return eng.run_heuristic(coords_float, spp, instance_cls, instance_box, instance_box_volume,
-                             instance_classes=instance_classes, rule=heuristic_rule,
-                             spp_align=(dataset_name == "scannetv2"), occ_thresh=0.7)
+    return _heuristic_one(coords_float, spp, instance_cls, instance_box, instance_box_volume, heuristic_rule,
+                          instance_classes, dataset_name)
+
+
+# method -> (rule for points in several boxes, occupancy a box needs to win a superpoint's vote)
+HEURISTIC_METHODS = {"box2mask": ("volume", None), "volume": ("volume", 0.7), "dist": ("dist", 0.7),
+                     "none": ("none", 0.7)}
+
+
+def _heuristic_one(coords_float, spp, instance_cls, instance_box, instance_box_volume, method, instance_classes,
+                   dataset_name):
+    scene = SceneInputs(coords_float, None, spp, instance_cls, instance_box, instance_box_volume)
+    return gen_pseudo_labels_heuristic_batch([scene], method=method, instance_classes=instance_classes,
+                                             dataset_name=dataset_name,
+                                             device=coords_float.device if coords_float.is_cuda else None)[0]
+
+
+def gen_pseudo_labels_heuristic_batch(scenes, method="box2mask", instance_classes=18, dataset_name="scannetv2",
+                                      device=None):
+    """Many scenes through ONE pass of the heuristic labelers.  `scenes` is a sequence of SceneInputs, of which only
+    coords_float, spp and the instance boxes / classes / volumes are read (no wall boxes, no floor slab).
+    method "box2mask" labels as gen_pseudo_label_box2mask, "volume" / "dist" / "none" as gen_pseudo_label with
+    that heuristic_rule; for scannetv2 the labels are aligned to superpoints, otherwise (s3dis) they stay per point.
+    Returns one (ps_semantic_label[N] int32, ps_instance_label[N] int32) pair per scene."""
+    if method not in HEURISTIC_METHODS:
+        raise ValueError(f"unknown heuristic method {method!r}; expected one of {sorted(HEURISTIC_METHODS)}")
+    rule, occ_thresh = HEURISTIC_METHODS[method]
+    eng = get_engine(device)
+    return eng.run_heuristic(list(scenes), rule=rule, spp_align=(dataset_name == "scannetv2"), occ_thresh=occ_thresh,
+                             instance_classes=instance_classes)
 
 
 # --------------------------------------------------------------------------------------------

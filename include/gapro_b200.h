@@ -156,6 +156,21 @@ int gapro_multibox_sources(const double* xyz, const int64_t* pt_off_dev, const i
                            const float* boxes, int32_t n_scenes, int64_t n_points, int32_t* dist_src, void* ws,
                            size_t ws_bytes, void* stream);
 
+/* Final labels of the heuristic labelers for a whole batch (gen_ps_utils.py:283-288 / :559-564), one launch.
+ * Reads the scene-local results of gapro_heuristic_labels: box index b >= 0 -> sem = boxes_cls[box_off[scene] + b],
+ * inst = b; -1 (background) -> sem = instance_classes, inst = -100; -2 (undecided, rule "none") -> both -100.
+ *   box_off_dev dev int32[n_scenes+1]; boxes_cls dev int64[box_off[n_scenes]] (the scenes' instance classes)
+ *   spp_align  1: inst_spp dev int32[s_total], spp_off_dev dev int32[n_scenes+1] -> packed_spp dev int32[s_total,4]
+ *              (16-byte aligned) receives the records (sem, inst, 1.0f bits, 0) of gapro_broadcast_labels;
+ *              inst_pt, pt_off_dev, sem, inst unused
+ *              0: inst_pt dev int32[n_points], pt_off_dev dev int64[n_scenes+1] -> sem, inst dev int32[n_points];
+ *              inst_spp, spp_off_dev, packed_spp unused
+ */
+int gapro_heuristic_finalize(const int32_t* inst_spp, const int32_t* inst_pt, const int32_t* spp_off_dev,
+                             const int64_t* pt_off_dev, const int32_t* box_off_dev, const int64_t* boxes_cls,
+                             int32_t instance_classes, int32_t n_scenes, int32_t s_total, int64_t n_points,
+                             int32_t spp_align, void* packed_spp, int32_t* sem, int32_t* inst, void* stream);
+
 /* ---------------------------------------------------------------------------
  * B — superpoint feature pooling.  Replaces
  *     gp_feats_spp = torch_scatter.scatter(gp_feats, spp, dim=0, reduce="mean")   gen_ps_utils.py:357
