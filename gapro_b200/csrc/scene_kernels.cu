@@ -894,10 +894,15 @@ extern "C" int gapro_pool_feats(const float* feats, const int32_t* perm, const i
     GAPRO_REQUIRE(s_total > 0 && D > 0, "gapro_pool_feats: empty input");
     GAPRO_REQUIRE(D <= 64, "gapro_pool_feats: feature dimension %d > 64", D);
     const size_t smem = (size_t)POOL_WARPS * 32 * D * sizeof(float);
-    static bool attr = false;
-    if (!attr) {
+    // cudaFuncSetAttribute is per device: D > 48 needs more than 48 KB of dynamic shared memory on every device the
+    // process pools on
+    static bool attr_done[64] = {};
+    int dev = 0;
+    GAPRO_CUDA_TRY(cudaGetDevice(&dev));
+    GAPRO_REQUIRE(dev >= 0 && dev < 64, "gapro_pool_feats: device ordinal %d not supported", dev);
+    if (!attr_done[dev]) {
         GAPRO_CUDA_TRY(cudaFuncSetAttribute(k_pool_feats<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-        attr = true;
+        attr_done[dev] = true;
     }
     const unsigned grid = (unsigned)((s_total + POOL_WARPS - 1) / POOL_WARPS);
     if (D == 6)
